@@ -145,6 +145,24 @@ def _build(P, cfg, cfg_name, sampling_steps):
                            pretrained_pth="", **cfg["unet_kw"])
 
 
+DUMP_BYTES = 60 * 2 ** 20     # --dump-outputs: float32 bytes written in all, split evenly over the arrays
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy (float32).  An array over its share of DUMP_BYTES is written as the 1-D
+    vector of its elements at a fixed set of flat indices (seeded permutation, ascending), the same for every run."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // 4 // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float()
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            a = a.reshape(-1)[idx.to(a.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.cpu().numpy())
+
+
 def cpu_baseline(threads=None, cfg_name="mug128", sampling_steps=None):
     """The reference's CPU arithmetic (oracle port, bit-exact vs the reference on this path) on a bounded sample:
     B=1, F=8-frame probe first; if the box is fast enough 2 full 40-frame UNet evals, else the probe scaled by 5;
@@ -254,7 +272,12 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="samples per GPU (default: the config's, 8 for config 2)")
     ap.add_argument("--sampling-steps", type=int, default=0, help="default: the config's (1000 DDPM for config 2)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the last step's outputs (sample_out_vid, sample_warped_vid, "
+                         "sample_vid_grid, sample_vid_conf; a seeded sample of the larger ones) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     cfg = CONFIGS[args.config]
     args.sampling_steps = args.sampling_steps or cfg["steps"]
     if args.strong:
@@ -332,7 +355,11 @@ def main():
     t_dev = timed(args.steps, False)
     clocks = sampler.stop() if rank == 0 else None
     seng = model.diffusion._engine()
-    t_e2e = timed(max(3, min(args.steps, 5)), True)          # >= 3 end-to-end samples, median
+    t_e2e = timed(args.steps, True)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {
+            "sample_out_vid": gather if world > 1 else model.sample_out_vid, "sample_warped_vid": model.sample_warped_vid,
+            "sample_vid_grid": model.sample_vid_grid, "sample_vid_conf": model.sample_vid_conf})
 
     ms = sum(t_dev) / len(t_dev)
     ms_e2e = sorted(t_e2e)[len(t_e2e) // 2]

@@ -4,10 +4,9 @@ A clean-room, CPU, fp32 restatement of the LFDM sampling + decode hot path (SURV
 written functionally over a flat ``state_dict`` (the reference's own key names), so the same
 weights can be fed to the reference, to this oracle and to the CUDA path.
 
-Parity status: PINNED against the unmodified reference executed in this container through
-``oracle/ref_shim.py`` (tests/test_oracle_vs_reference.py, run whenever /root/reference exists)
-and against the committed golden fixtures under tests/golden/ (generated from the reference by
-``oracle/make_golden.py``).  The third-party rotary embedding (rotary_embedding_torch==0.1.5,
+Parity status: PINNED against the unmodified reference, executed through ``oracle/ref_shim.py``
+to generate the committed golden fixtures under tests/golden/ (``oracle/make_golden.py``,
+``oracle/make_golden_reference.py``; tests/test_oracle_golden.py, tests/test_oracle_vs_reference.py).  The third-party rotary embedding (rotary_embedding_torch==0.1.5,
 not vendored in the reference) is restated from its published algorithm: that one boundary is
 "parity unpinned" (no reference test or vector pins the interleaved-pair convention).
 

@@ -6,6 +6,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+# PyTorch splits the CPU oracle's convolution / matmul sums over its intra-op threads, so their rounding depends on the
+# thread count; the vectors under tests/golden/ were recorded with 8 threads and several tests compare bit for bit
+GOLDEN_THREADS = 8
 
 
 def pytest_configure(config):
@@ -20,6 +23,15 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords:
             item.add_marker(skip)
+
+
+@pytest.fixture(autouse=True)
+def golden_threads():
+    import torch
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 @pytest.fixture(scope="session")

@@ -1,39 +1,22 @@
 """CPU: text conditioning (cvpr23_lfdm_b200/dm/text.py) -- the reference's pooling arithmetic on an injected tiny BERT, the
 label-table path, and the failure mode when neither weights nor table are available."""
-import importlib.util
-import os
 import pytest
 import torch
 
-REF_TEXT = "/root/reference/DM/modules/text.py"
 
-
-def _tiny_bert():
-    from transformers import BertConfig, BertModel
-    torch.manual_seed(3)
-    cfg = BertConfig(vocab_size=50, hidden_size=32, num_hidden_layers=2, num_attention_heads=2, intermediate_size=64,
-                     max_position_embeddings=32)
-    return BertModel(cfg).eval()
-
-
-def test_bert_embed_matches_reference_pooling():
-    """same model, same padded token ids -> identical masked mean (excluding [CLS]) and [CLS] outputs as the reference"""
-    if not os.path.exists(REF_TEXT):
-        pytest.skip("reference checkout not present")
+def test_bert_embed_matches_reference_pooling(golden):
+    """same model, same padded token ids -> identical masked mean (excluding [CLS]) and [CLS] outputs as the reference
+    (recorded by oracle/make_golden_reference.py)"""
     from cvpr23_lfdm_b200.dm import text as T
-    spec = importlib.util.spec_from_file_location("ref_text", REF_TEXT)
-    R = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(R)
-    bert = _tiny_bert()
-    R.MODEL, T.MODEL = bert, bert
+    from oracle.make_golden_reference import tiny_bert
+    g = golden("reference_checks.pt")["bert"]
+    T.MODEL = tiny_bert()
     try:
-        ids = torch.tensor([[2, 7, 9, 11, 3, 0, 0], [2, 5, 3, 0, 0, 0, 0], [2, 4, 6, 8, 10, 12, 3]])
-        for cls in (False, True):
-            ref = R.bert_embed(ids, return_cls_repr=cls)
-            got = T.bert_embed(ids, return_cls_repr=cls)
+        for cls, ref in ((False, g["mean"]), (True, g["cls"])):
+            got = T.bert_embed(g["ids"], return_cls_repr=cls)
             assert torch.equal(ref, got)
     finally:
-        R.MODEL, T.MODEL = None, None
+        T.MODEL = None
 
 
 def test_label_table_roundtrip_and_missing_label(tmp_path):
